@@ -9,6 +9,8 @@ all-reduce, dense SGD) at global batch 65536 and prints ONE JSON line from rank 
 * ``e2e``: the same metric through the public API with the per-step host->device copy of the
   inputs from pinned memory and the device->host read of the loss inside the timed region.
 * ``--impl reference`` reports the unmodified reference (TensorFlow + Horovod) if importable.
+* ``--dump-outputs DIR`` writes what the last timed step computed as ``.npy`` files; the inputs
+  are seeded, so two builds run with the same flags can be compared output for output.
 
 Reference counterpart: examples/dlrm/main.py + examples/benchmarks/synthetic_models/main.py
 (host wall-clock timing, :132-158); BASELINE.md for the published 8xA100 numbers.
@@ -30,6 +32,7 @@ sys.path.insert(0, ROOT)
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 BASELINE_SAMPLES_PER_SEC = 10416232.0  # 8xA100 AMP, reference examples/dlrm/README.md:8
+DUMP_ROWS = 256  # batch positions whose embedding rows --dump-outputs writes (per table)
 
 
 def parse_args():
@@ -74,6 +77,11 @@ def parse_args():
   p.add_argument("--no-verify", action="store_true",
                  help="skip the pre-flight numerics check (2 steps of a 1/1000-rows plan on all "
                       "ranks vs a single-process fp32 PyTorch oracle on rank 0)")
+  p.add_argument("--dump-outputs", default=None, metavar="DIR",
+                 help="write what the last timed step computed to DIR/<name>.npy: its loss, the "
+                      "dense parameters after its update and the updated embedding rows at "
+                      f"{DUMP_ROWS} seeded positions of its batch (float32, their ids float64), "
+                      "to compare two builds output for output")
   return p.parse_args()
 
 
@@ -210,6 +218,52 @@ def gen_ids(rows: int, n: int, alpha: float, gen):
   g = 1.0 - alpha
   y = (r * ((rows + 1.0)**g - 1.0) + 1.0)**(1.0 / g)
   return (y.to(torch.int64) - 1).clamp_(0, rows - 1).to(torch.int32)
+
+
+def step_outputs(model, loss, cat, world, rank):
+  """Device copies of what a training step computed: the mean loss over ranks, the dense
+  parameters and the embedding rows looked up at DUMP_ROWS seeded positions of rank 0's batch
+  ``cat`` ([tables, batch] ids), read from whichever rank owns each piece.  Collective at
+  world > 1; rank 0 gets a dict of float tensors, the other ranks None."""
+  import torch
+  import torch.distributed as dist
+  emb = model.embedding
+  st, dev = emb.strategy, cat.device
+  loss = loss.detach().float().reshape(1).clone()
+  pos = torch.randperm(cat.shape[1], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS]
+  ids = cat[:, pos.to(dev)].long().contiguous()
+  if world > 1:
+    dist.all_reduce(loss)
+    loss /= world
+    dist.broadcast(ids, src=0)
+  # the global tables are split into replicated, column-sliced and row-sliced groups; every
+  # (row, column) has one owner, which copies it in, and a sum over ranks assembles the rows
+  weights = emb.weights
+  n_dp, n_col = len(emb.dp_layers), len(emb.local_embedding_layers)
+  rows = torch.zeros(ids.shape[0], ids.shape[1], model.embedding_dim, device=dev)
+
+  def take(w, i):
+    return w.detach().index_select(0, i.to(w.device)).to(dev, torch.float32)
+
+  if rank == 0:
+    for t, w in zip(st.table_groups[0], weights[:n_dp]):
+      rows[t] = take(w, ids[t])
+  for s in st.shards[rank]:
+    t = st.table_groups[1][s.table]
+    rows[t, :, s.col_start:s.col_end] = take(weights[n_dp + s.local_table], ids[t] + s.row_offset)
+  for gt, t in enumerate(st.table_groups[2]):
+    lo, hi = st.row_ranges[gt][rank]
+    mine = (ids[t] >= lo) & (ids[t] < hi)
+    rows[t, mine] = take(weights[n_dp + n_col + gt], ids[t][mine] - lo)
+  if world > 1:
+    dist.reduce(rows, dst=0)
+  if rank != 0:
+    return None
+  out = {"loss": loss, "embedding_rows": rows, "embedding_row_ids": ids.double()}
+  for name, p in model.named_parameters():
+    if not name.startswith("embedding."):
+      out[name] = p.detach().float().clone()
+  return out
 
 
 def verify(args, device, world, rank, compute_dtype, cst_for):
@@ -527,17 +581,19 @@ def main():
       torch.cuda.synchronize()
 
   def timed(fn, steps):
+    """Milliseconds for ``steps`` calls of ``fn`` (max over ranks) and the last call's result."""
     sync_all()
     start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    result = None
     start.record()
     for i in range(steps):
-      fn(i)
+      result = fn(i)
     end.record()
     sync_all()
     ms = torch.tensor([start.elapsed_time(end)], device=device)
     if world > 1:
       dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    return float(ms.item())
+    return float(ms.item()), result
 
   for i in range(max(3, args.warmup)):
     step_from_device(i)
@@ -545,8 +601,13 @@ def main():
   if rank == 0:
     sampler.start()
   _native.reset_launch_count()
-  total_ms = timed(step_from_device, args.steps)
+  total_ms, last_loss = timed(step_from_device, args.steps)
   launches = _native.launch_count()
+  dumped = None
+  if args.dump_outputs:
+    # taken before anything else runs a step (the launch count below runs one more)
+    last_batch = (dev_i[0] - 1 if use_fast else args.steps - 1) % len(dev_pool)
+    dumped = step_outputs(model, last_loss, dev_pool[last_batch][1], world, rank)
   if use_fast and args.cuda_graph:
     # kernels replayed from the captured graph are not seen by the python-side counter:
     # count one eager pass of the same schedule
@@ -605,12 +666,17 @@ def main():
     else:
       for i in range(3):
         step_e2e(i)
-    e2e_ms = timed(step_e2e, args.steps)
+    e2e_ms, _ = timed(step_e2e, args.steps)
     e2e = {"value": gb * args.steps / (e2e_ms / 1e3), "unit": "samples/s",
            "ms_per_step": e2e_ms / args.steps, "h2d_bytes_per_step": h2d_bytes * world,
            "d2h_bytes_per_step": 4 * world}
   if engine is not None:
     engine.ctx.check_errors()
+  if dumped is not None:
+    import numpy as np
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for name, t in dumped.items():
+      np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.cpu().numpy())
 
   if rank == 0:
     ms_per_step = total_ms / args.steps
